@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — latent-frames/sec through the full GCD denoising hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload kubric|pardom|direct50]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload kubric|pardom|direct50] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one batch: per GPU ONE clip of 14 latent frames, 72x128 (576x1024 px):
 25 EDM/Euler steps of the CFG-doubled SVD VideoUNet (28 frames per forward) + the temporal VAE decode of the 14 frames
@@ -15,6 +15,9 @@ device->host read of the decoded frames inside the timed region; `roofline` = te
 class (tc_gemm implicit-GEMM conv/linear) from CUDA events on the launching stream + whole-path fraction; `cpu_baseline` =
 the CPU oracle port (oracle/gcd_oracle.py) timed on this box's host cores on a bounded sample.
 `--impl reference` times only that CPU port (the reference's own PyTorch code cannot travel to the GPU box).
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as float32 .npy files, for comparing two builds on
+identical seeded inputs: latents.npy [14, 4, h, w]; frames.npy, or frames_sample.npy (a fixed seeded sample of 2^23
+values of the flattened [14, 3, 8h, 8w] frames) when the frames exceed that; latents_gathered.npy [N, 14, 4, h, w] with N > 1.
 """
 import argparse
 import json
@@ -26,6 +29,7 @@ import time
 
 import torch
 
+sys.dont_write_bytecode = True       # the tree may be read-only; nothing is cached next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -285,11 +289,43 @@ def run_extra_workloads(args, wl, pipe, ust, dev, rank, world, lat, timed, gathe
     return out
 
 
+# ------------------------------------------------------------------------------------------------------ output dump
+DUMP_FRAMES_SAMPLE = 1 << 23          # float32 values: 32 MiB of the 99 MB of frames of a 576x1024 clip
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, z, frames, gathered):
+    """Writes the arrays of one timed step as float32 .npy files (see the module docstring); at most DUMP_LIMIT bytes."""
+    import numpy as np
+    arrays = {"latents": z}
+    if frames is not None:
+        if frames.numel() <= DUMP_FRAMES_SAMPLE:
+            arrays["frames"] = frames
+        else:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randperm(frames.numel(), generator=g)[:DUMP_FRAMES_SAMPLE].sort().values
+            arrays["frames_sample"] = frames.reshape(-1)[idx.to(frames.device)]
+    if gathered is not None:
+        arrays["latents_gathered"] = torch.stack(gathered)
+    total = sum(a.numel() * 4 for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach().float().cpu().numpy())
+
+
+def positive_int(v):
+    n = int(v)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return n
+
+
 # ------------------------------------------------------------------------------------------------------ product arm
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--steps", type=positive_int, default=2, help="timed steps (one clip per GPU each)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="kubric", choices=list(WORKLOADS))
@@ -297,6 +333,8 @@ def main():
     ap.add_argument("--no-decode", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--cpu-leg", default=None, help=argparse.SUPPRESS)
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_workloads block (BASELINE configs 3/4, CFG-parallel)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latents and frames of the last timed step (rank 0) to DIR/<name>.npy, float32")
     ap.add_argument("--profile-run", action="store_true",
                     help="for ncu: exactly --warmup/--steps resident steps, no e2e / instrumented / CPU passes, no JSON claims")
     args = ap.parse_args()
@@ -304,6 +342,8 @@ def main():
         return _cpu_leg_worker(args.cpu_leg)
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs the product arm: --impl reference only times the CPU port")
         return run_reference(args, wl)
 
     import torch.distributed as dist
@@ -345,6 +385,11 @@ def main():
             dist.all_gather(gathered, z.contiguous())     # the path's only collective: final gather over NVLink
         return z, fr
 
+    last = {}
+
+    def step_resident_kept():
+        last["z"], last["frames"] = step_resident()
+
     def step_e2e():
         z, fr = pipe.sample_video(hx, hc, huc, decode=not args.no_decode)
         if fr is not None:
@@ -383,9 +428,12 @@ def main():
         step_resident()
     clocks = ClockSampler(local) if rank == 0 else None
     l0 = ops.launch_count()
-    ms = timed(step_resident, args.steps)
+    ms = timed(step_resident_kept, args.steps)
     launches = ops.launch_count() - l0
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["z"], last["frames"], gathered)
+    last.clear()
     step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
 

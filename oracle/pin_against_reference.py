@@ -5,7 +5,7 @@
 For each case the REFERENCE's own modules (imported through oracle/ref_shim.py) are run on CPU fp32 with seeded
 weights/inputs (oracle/weights.py); the golden tensors stored are the reference outputs, and the oracle restatement is
 asserted to agree with them (max-abs relative to output scale < 2e-5). Also dumps the reference state-dict key/shape
-lists used by tests/test_spec_cpu.py. `--full` adds the full-width Kubric architecture (1.5 B parameters).
+lists used by tests/test_spec_cpu.py and the reference helpers' view of the modules (host_api.json). `--full` adds the full-width Kubric architecture (1.5 B parameters).
 """
 import json
 import os
@@ -140,6 +140,59 @@ def pin_embedders():
     torch.save(out, os.path.join(GOLD, "embedders.pt"))
 
 
+def pin_host_api():
+    """What the reference's host-side helpers make of this package's modules, so the tests need no reference tree:
+    the LitEma shadow names of `HotPathRoot.model` (modules/ema.py) and the embedder attributes the GeneralConditioner
+    reads and sets (encoders/modules.py:40-81, 93-130). The two conditioner classes are cut out of the reference source
+    with `ast` and executed against the repo's embedders, as in ref_shim.ref_embedder_classes."""
+    import ast
+    import importlib
+    import types
+    import typing
+    import torch.nn as nn
+    from gcd_b200 import checkpoint, spec
+    from gcd_b200.sampling import instantiate_from_config
+    from gcd_b200.unet import VideoUNet
+    from gcd_b200.vae import Encoder, VideoDecoder
+    ref_shim.install()
+    from sgm.modules.ema import LitEma
+    root = checkpoint.HotPathRoot(VideoUNet(**spec.unet_ctor_kwargs(spec.UNET_TINY)),
+                                  VideoDecoder(**spec.decoder_ctor_kwargs(spec.VAE_TINY)),
+                                  Encoder(**spec.encoder_ctor_kwargs(spec.VAE_ENCODER_TINY)))
+    out = {"litema_shadows_of_model": LitEma(root.model, decay=0.999).m_name2s_name}
+    path = os.path.join(ref_shim.REF, "sgm", "modules", "encoders", "modules.py")
+    body = [n for n in ast.parse(open(path).read()).body
+            if isinstance(n, ast.ClassDef) and n.name in ("AbstractEmbModel", "GeneralConditioner")]
+    ns = {"torch": torch, "nn": nn, "Union": typing.Union, "List": typing.List, "Dict": typing.Dict,
+          "Optional": typing.Optional, "ListConfig": list, "instantiate_from_config": instantiate_from_config,
+          "disabled_train": lambda self, mode=True: self, "count_params": lambda m, verbose=False: 0,
+          "print": lambda *a, **k: None}
+    exec(compile(ast.Module(body=body, type_ignores=[]), path, "exec"), ns)
+    base = ns["AbstractEmbModel"]
+    out["abstract_emb_model"] = {k: getattr(base(), k) for k, v in vars(base).items() if isinstance(v, property)}
+    fake = types.ModuleType("sgm.modules.encoders.modules")
+    fake.AbstractEmbModel = base
+    pkg = types.ModuleType("sgm.modules.encoders")
+    pkg.__path__ = []
+    sys.modules["sgm.modules.encoders"], sys.modules["sgm.modules.encoders.modules"] = pkg, fake
+    import gcd_b200.embedders as E
+    importlib.reload(E)
+    configs = [{"target": "gcd_b200.embedders.ConcatTimestepEmbedderND", "params": {"outdim": 256}, "input_key": "fps_id",
+                "is_trainable": False},
+               {"target": "gcd_b200.embedders.SphericalEmbedder", "params": {"embed_dim": 128}, "input_key": "spherical",
+                "is_trainable": False, "ucg_rate": 0.1}]
+    cond = ns["GeneralConditioner"](configs)
+    out["general_conditioner"] = [
+        {"config": cfg, "class": type(e).__name__, "input_key": e.input_key, "ucg_rate": e.ucg_rate,
+         "is_trainable": e.is_trainable, "legacy_ucg_val": e.legacy_ucg_val, "training": e.training,
+         "requires_grad": [p.requires_grad for p in e.parameters()]} for cfg, e in zip(configs, cond.embedders)]
+    del sys.modules["sgm.modules.encoders"], sys.modules["sgm.modules.encoders.modules"]
+    importlib.reload(E)
+    json.dump(out, open(os.path.join(GOLD, "host_api.json"), "w"), indent=0, sort_keys=True)
+    print(f"[host api] {len(out['litema_shadows_of_model'])} LitEma shadows; conditioner accepted "
+          f"{[d['class'] for d in out['general_conditioner']]}")
+
+
 def pin_closed_forms():
     """Known-answer values derivable from the source (SURVEY.md §8(c))."""
     ref_shim.install()
@@ -168,6 +221,7 @@ if __name__ == "__main__":
     pin_decoder("tiny", VAE_TINY, T=3, H=8, W=8)
     pin_encoder("tiny", dict(O.VAE_ENCODER, ch=64), n=2, H=64, W=96)
     pin_embedders()
+    pin_host_api()
     if "--full" in sys.argv:
         pin_unet("kubric", O.UNET_KUBRIC, B=1, T=2, H=16, W=16, steps=2)
         pin_unet("pardom", O.UNET_PARDOM, B=1, T=2, H=8, W=8, steps=1)

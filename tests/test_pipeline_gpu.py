@@ -196,6 +196,30 @@ def test_sampler_50_steps_scale_2p5_fused_equals_generic():
     assert relerr(b, a) < 1e-2
 
 
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the last timed step's latents and frames as float32 .npy; two runs with the same
+    arguments sample the same seeded inputs, so their dumps agree to the run-to-run noise of the fp64 statistics atomics."""
+    import json
+    import subprocess
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "0",
+                            "--workload", "tiny-selftest", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 2
+        dumps.append({n: np.load(d / f"{n}.npy") for n in ("latents", "frames")})
+        assert sorted(os.listdir(d)) == ["frames.npy", "latents.npy"]
+    for n, shape in (("latents", (14, 4, 16, 24)), ("frames", (14, 3, 128, 192))):
+        a, b = dumps[0][n], dumps[1][n]
+        assert a.dtype == np.float32 and a.shape == shape and np.isfinite(a).all() and np.abs(a).max() > 0
+        assert np.linalg.norm(a - b) / np.linalg.norm(b) < 1e-4, n
+
+
 def test_cfg_parallel_two_gpus():
     """SURVEY.md §8(f) rank 2 on real hardware (skipped on a 1-GPU box): one clip over two GPUs (uc | c) with NCCL equals the
     single-GPU fused sampler within the 16-bit noise floor and leaves both ranks with bit-identical latents."""
